@@ -9,7 +9,7 @@ replicated weights (configs[3]), no data-path collective; weak scaling.
 
   value  whole-job audio seconds / device-timed seconds, PCM already resident in HBM
   e2e    the same metric through the public C API with HOST PCM (H2D of the PCM and D2H of the token
-         ids inside the timed region)
+         ids inside the timed region), one pass after the timed steps
   roofline  decode step (the dominant phase, >90% of the time): algorithmic bytes per step
          (6.858 GB bf16 weights + f32 KV rows read) / device time per step, vs MEASURED_PEAKS.json
   cpu_baseline  the UNMODIFIED reference (oracle/_ref, built from /root/reference by oracle/Makefile)
@@ -24,7 +24,11 @@ replicated weights (configs[3]), no data-path collective; weak scaling.
   sharded_encoder  (N > 1) one 1-hour recording, encoder sharded by sequence over the N GPUs in host C with NCCL
          (vox_cuda_encode_sharded: per-layer K/V halo ncclSend/ncclRecv + adapter ncclAllGather), vs the same call unsharded
 
-`--impl reference` times only that CPU reference arm.  The model is the seeded synthetic checkpoint
+`--steps K --warmup W` run max(W, 3) untimed and K timed passes; the e2e pass follows.  cpu_baseline, multistream, live and
+sharded_encoder are the extra legs: they run with `--extra-legs` and are null otherwise.
+`--impl reference` times only that CPU reference arm.  `--dump-outputs DIR` writes what the last timed step returned to its
+caller (token ids, unit counts) as DIR/<name>.npy in float64, so that two builds can be compared output for output: the
+synthetic checkpoint and PCM are seeded, so the inputs are identical from run to run.  The model is the seeded synthetic checkpoint
 (tools/make_synth_model.c): there is no network for the real weights; throughput does not depend on them.
 """
 import argparse
@@ -43,18 +47,25 @@ sys.path.insert(0, ROOT)
 
 WEIGHT_BYTES_PER_STEP = 2 * (26 * 116_391_936 + 131072 * 3072)      # bf16 matrices streamed by one decode step
 KV_BYTES_PER_SLOT = 26 * 1024 * 4 * 2                                 # f32 K and V rows, all layers
-SYNTH_DIR = os.environ.get("VOX_SYNTH_DIR", "/dev/shm/voxsynth_b200")
+
+
+T_START = time.perf_counter()
 
 
 def log(*a):
     print(*a, file=sys.stderr, flush=True)
 
 
+def phase(name):
+    """Progress on stderr: a run that is stopped early still shows how far it got."""
+    log(f"bench: {name} ({time.perf_counter() - T_START:.1f} s)")
+
+
 def ensure_inputs(seconds):
     sys.path.insert(0, os.path.join(ROOT, "tests"))
     from conftest import ensure_synth_model, read_wav_f32, synth_wav
-    model = ensure_synth_model(SYNTH_DIR)
-    pcm = read_wav_f32(synth_wav(seconds, SYNTH_DIR))
+    model = ensure_synth_model()
+    pcm = read_wav_f32(synth_wav(seconds))
     return model, pcm
 
 
@@ -215,7 +226,11 @@ def main():
     ap.add_argument("--live-seconds", type=float, default=15.0, help="length of the 0.1-s live-feeding leg (N=1 only; 0 = skip)")
     ap.add_argument("--streams", type=int, default=8, help="streams per GPU in the multistream leg (N=1 only; 1 = skip)")
     ap.add_argument("--sharded-seconds", type=float, default=3600.0, help="recording length of the sharded-encoder leg (N>1)")
+    ap.add_argument("--extra-legs", action="store_true", help="also run cpu_baseline, multistream, live and sharded_encoder")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the outputs of the last timed step as DIR/<name>.npy (float64)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     rank = int(os.environ.get("RANK", "0")); world = int(os.environ.get("WORLD_SIZE", "1"))
     local = int(os.environ.get("LOCAL_RANK", "0"))
     n_gpus = max(args.gpus, world)
@@ -263,14 +278,17 @@ def main():
         ensure_inputs(args.seconds)
     barrier()
     model, pcm = ensure_inputs(args.seconds)
+    phase("inputs ready")
     import vbload
     vb = vbload.load()
     multi = vbload.load_submodule("multi")
     t_load = time.perf_counter()
     eng = vb.Engine(model)
     load_s = time.perf_counter() - t_load
+    phase("engine loaded")
     d_pcm = eng.to_device(pcm)
     profiling = os.environ.get("VOX_BENCH_PROFILE") == "1"      # ncu runs: fewer warm-ups, no extra legs (never a bench value)
+    extra = args.extra_legs and not profiling
 
     def one_pass(device_input):
         s = eng.stream()
@@ -302,12 +320,17 @@ def main():
     n_warm = args.warmup if profiling else max(args.warmup, 3)
     for _ in range(n_warm):
         ids, counts = one_pass(True)
+    phase("warm-up done")
     sampler = ClockSampler(local); sampler.start()
     i_before = eng.info()
     dev_ms, _, (ids, counts) = timed(args.steps, lambda: one_pass(True))
     i_after = eng.info()
     sampler.stop.set(); sampler.join(timeout=3)
-    e2e_ms, e2e_wall, (ids2, _) = timed(args.steps, lambda: one_pass(False))
+    if rank == 0 and args.dump_outputs:
+        dump_outputs(args.dump_outputs, ids, counts)
+    phase("timed steps done")
+    e2e_ms, e2e_wall, (ids2, _) = timed(1, lambda: one_pass(False))
+    phase("host-PCM pass done")
 
     # the work that was timed is the work the reference would do on this recording (an early EOS would shrink it silently)
     assert (counts["mel_frames"], counts["adapter_tokens"], len(ids)) == (frames, toks, steps_expected), \
@@ -315,7 +338,7 @@ def main():
 
     audio_s = args.seconds * args.steps * world
     value = audio_s / (dev_ms / 1e3)
-    e2e_value = audio_s / max(e2e_ms / 1e3, e2e_wall)
+    e2e_value = args.seconds * world / max(e2e_ms / 1e3, e2e_wall)
     dsteps = i_after["total_decode_steps"] - i_before["total_decode_steps"]
     dms = i_after["total_decode_kernel_ms"] - i_before["total_decode_kernel_ms"]
     n_dec = len(ids)
@@ -368,7 +391,7 @@ def main():
 
     # ---- several streams per weight pass on this GPU (N = 1 only: the scaling run keeps one stream per GPU)
     ms_block = None
-    if world == 1 and not profiling and args.streams > 1:
+    if world == 1 and extra and args.streams > 1:
         B = args.streams
         forks = [eng.fork() for _ in range(B - 1)]
         engines = [eng] + forks
@@ -407,8 +430,9 @@ def main():
             f.close()
 
     # ---- live shape (main.c --stdin -I 0.1 / --from-mic): 0.1 s feeds, one small encoder call + 1-2 decode steps per feed
+    phase("multistream leg done")
     live = None
-    if world == 1 and not profiling and args.live_seconds > 0:
+    if world == 1 and extra and args.live_seconds > 0:
         n_live = min(pcm.size, int(args.live_seconds * 16000))
         for rep in range(2):                                   # first repetition warms the small-M workspaces
             st = eng.stream()
@@ -433,11 +457,13 @@ def main():
 
     # ---- one long recording, encoder sharded over the ranks (N > 1)
     sharded = None
-    if world > 1 and not profiling:
+    if world > 1 and extra:
         sharded = sharded_encoder_leg(vb, eng, dist, rank, world, local, multi, args.sharded_seconds)
 
     if rank == 0:
-        cpu = reference_sample(model, args.seconds) if (world == 1 and not profiling) else None
+        phase("live leg done")
+        cpu = reference_sample(model, args.seconds) if (world == 1 and extra) else None
+        phase("host reference sample done")
         traffic, traffic_src = ncu_traffic()
         line = {
             "metric": "real-time factor (audio-s/wall-s)", "value": value, "unit": "x real-time", "n_gpus": n_gpus,
@@ -477,6 +503,15 @@ def main():
     eng.close()
     if dist is not None:
         dist.destroy_process_group()
+
+
+def dump_outputs(out_dir, ids, counts):
+    """The arrays vox_stream_* hands its caller for the benchmarked recording: the greedy token ids and the unit counts
+    (mel frames, adapter tokens, decoder steps).  Integers, stored as float64 (exact)."""
+    os.makedirs(out_dir, exist_ok=True)
+    np.save(os.path.join(out_dir, "token_ids.npy"), np.asarray(ids, dtype=np.float64))
+    np.save(os.path.join(out_dir, "counts.npy"),
+            np.array([counts["mel_frames"], counts["adapter_tokens"], counts["decoder_steps"]], dtype=np.float64))
 
 
 def sharded_encoder_leg(vb, eng, dist, rank, world, local, multi, seconds):
